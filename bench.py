@@ -9,6 +9,7 @@ policy rollout only.  N>1: weak scaling, 4096 envs per GPU, no data-path collect
   python bench.py --gpus 1 --steps 20 --warmup 3
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference          # the reference's CPU path: oracle port (fp64 C) on all host cores
+  python bench.py --dump-outputs DIR         # also write what the last timed step computed, DIR/<name>.npy, to compare two builds
 """
 import argparse
 import json
@@ -27,6 +28,7 @@ ENVS_PER_GPU = 4096
 CLIP_FRAMES = 320                      # length of '0-ACCAD_Male2General_c3d_A2- Sway_poses', the clip configs[1] names
 BYTES_PER_ENV_STEP = 6396              # algorithmic HBM bytes of the fused physics/task step, SURVEY.md section 8(d)
 METRIC, UNIT = "env_steps_per_s", "env-steps/s"
+DUMP_LIMIT = 64 << 20                  # bytes, all --dump-outputs arrays together
 
 
 def make_clip(seed=1):
@@ -34,6 +36,20 @@ def make_clip(seed=1):
     ex = motion_lib.synthetic_clip(CLIP_FRAMES, np.random.default_rng(seed))
     shape = np.zeros(17)
     return ex, shape
+
+
+def dump_outputs(path, arrays):
+    """DIR/<name>.npy for each array (tensor or numpy; float64 kept, everything else as float32), at most DUMP_LIMIT bytes in all."""
+    out = {}
+    for k, v in arrays.items():
+        a = v.detach().cpu().numpy() if hasattr(v, "detach") else np.asarray(v)
+        out[k] = a if a.dtype == np.float64 else a.astype(np.float32)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------ CPU reference arm
@@ -254,6 +270,12 @@ def run_gpu(args):
     if world > 1:
         dist.barrier()
     t_wall1 = time.time()
+    last = None
+    if args.dump_outputs and rank == 0:                  # the last timed step's results, copied before the steps below overwrite them
+        r = (K - 1) % R
+        last = dict(next_obs=agent.obs, state=buf.states[r], action=buf.actions[r], logp=buf.logp[r], reward=buf.rewards[r], mask=buf.masks[r],
+                    fail=buf.fails[r], obs_filter_stats=agent.running_state.stats)
+        last = {k: v.cpu() for k, v in last.items()}
     clk = clocks.stop(t_wall0, t_wall1) if clocks else None
     total_ms = sum(a.elapsed_time(b) for a, b in ev)
     ms = C.c_float(0)
@@ -286,7 +308,7 @@ def run_gpu(args):
 
     # end to end through host buffers: the step's input (the observations) comes from pinned host memory, the step runs through the public
     # call (BatchedAgent.rollout -> uhc_rollout), and its results (next obs, actions, reward, mask, fail) are read back to the host; one sync per step
-    Ke = max(3, min(K, 20))
+    Ke = K
     pin = lambda *shape, dtype=torch.float32: torch.empty(*shape, dtype=dtype).pin_memory()
     obs_h, act_h, rew_h, mask_h, fail_h = pin(E, 657), pin(E, 105), pin(E), pin(E), pin(E, dtype=torch.int32)
     obs_h.copy_(agent.obs)
@@ -346,6 +368,8 @@ def run_gpu(args):
                 env_counters=counters, clocks=clk)
     if cb:
         line["cpu_baseline"] = cb
+    if last:
+        dump_outputs(args.dump_outputs, last)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -417,6 +441,9 @@ def run_train(args):
     if world > 1:
         dist.barrier()
     t_wall1 = time.time()
+    if args.dump_outputs and rank == 0:                  # the parameters and observation statistics after the last iteration, and its losses
+        dump_outputs(args.dump_outputs, dict(policy_params=agent.policy.flat, value_params=agent.value.flat, obs_filter_stats=agent.running_state.stats,
+                                             losses=np.array([out["surr_loss"], out["value_loss"]], np.float32)))
     clk = clocks.stop(t_wall0, t_wall1) if clocks else None
     total_ms = ev[0].elapsed_time(ev[2 * K])
     sample_ms = sum(ev[2 * k].elapsed_time(ev[2 * k + 1]) for k in range(K)) / K
@@ -482,7 +509,14 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="rollout", choices=["rollout", "train"],
                     help="rollout (default, the headline: BASELINE configs[1]) or train (configs[2] at N=1, configs[3]/[4] shapes at N>1)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0's envs) as DIR/<name>.npy: float32 / float64, at most 64 MB; "
+                         "the same arguments give the same inputs, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl ours)")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "train":

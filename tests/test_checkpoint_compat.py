@@ -1,16 +1,15 @@
 """CPU: the checkpoint wire format (agent_copycat.py:190-201, :249-260).  `running_state` is a pickled
 uhc.khrylib.utils.zfilter.ZFilter; a file written by this repo must load into the REFERENCE's class and a file written by the reference
-must load here.  The cross-check against the real reference runs where a checkout exists ($UHC_REFERENCE, default /root/reference)."""
+must load here.  The cross-checks against the reference compare with what its own code wrote (tests/golden, tools/make_golden.py compat)."""
+import io
 import os
 import pickle
 import subprocess
 import sys
 
 import numpy as np
-import pytest
 
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
-REF = os.environ.get("UHC_REFERENCE", "/root/reference")
 
 
 def test_host_zfilter_matches_running_statistics():
@@ -28,46 +27,49 @@ def test_host_zfilter_matches_running_statistics():
     assert z3.rs._n == 50 and np.allclose(z3.rs._M, z2.rs._M) and np.allclose(z3.rs._S, z2.rs._S) and z3.clip == 5.0
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "uhc", "khrylib", "utils", "zfilter.py")), reason="no reference checkout on this machine")
-def test_running_state_round_trips_through_the_reference_class(tmp_path):
+class _ClassRecorder(pickle.Unpickler):
+    """unpickles into this repo's classes and records the ones from `uhc` the file names"""
+    def find_class(self, module, name):
+        if module.split(".")[0] == "uhc":
+            self.names.add((module, name))
+        return super().find_class(module, name)
+
+
+def _classes(data):
+    u = _ClassRecorder(io.BytesIO(data))
+    u.names = set()
+    return u.load(), u.names
+
+
+def _layout(o):
+    """attribute names, recursively through the `uhc` objects"""
+    return {k: _layout(v) if type(v).__module__.split(".")[0] == "uhc" else None for k, v in vars(o).items()}
+
+
+def test_running_state_round_trips_through_the_reference_class(golden_dir):
+    """tests/golden/zfilter_roundtrip.npz (tools/make_golden.py compat): a running_state pickled by the reference's own ZFilter, and what the
+    reference's ZFilter computed after loading this repo's pickle of the same statistics.  Ours must name the same classes with the same
+    attribute layout (so that it loads into the reference's), normalise as the reference did, and the reference's file must load here."""
     from uhc.khrylib.utils.zfilter import ZFilter
-    rng = np.random.RandomState(1)
-    x = rng.normal(0.5, 3.0, (40, 657))
+    g = np.load(os.path.join(golden_dir, "zfilter_roundtrip.npz"))
+    x = np.random.RandomState(1).normal(0.5, 3.0, (40, 657))
     ours = ZFilter.from_stats(40, x.mean(0), ((x - x.mean(0)) ** 2).sum(0), clip=5.0)
-    p1, p2 = tmp_path / "ours.p", tmp_path / "ref.p"
-    pickle.dump({"running_state": ours}, open(p1, "wb"))
-    np.save(tmp_path / "x.npy", x)
-    # in a clean interpreter with ONLY the reference on the path: load our pickle into the reference's class, use it, write one of its own
-    code = f"""
-import sys, pickle, numpy as np
-sys.path.insert(0, {REF!r})
-from uhc.khrylib.utils import zfilter
-assert zfilter.__file__.startswith({REF!r})
-cp = pickle.load(open({str(p1)!r}, 'rb'))
-rs = cp['running_state']
-assert type(rs).__module__ == 'uhc.khrylib.utils.zfilter' and rs.rs.n == 40
-x = np.load({str(tmp_path / 'x.npy')!r})
-y = rs(x[0], update=False)
-np.save({str(tmp_path / 'y.npy')!r}, y)
-z = zfilter.ZFilter((657,), clip=5)
-for r in x: z(r)
-pickle.dump({{'running_state': z}}, open({str(p2)!r}, 'wb'))
-"""
-    env = {k: v for k, v in os.environ.items() if k != "PYTHONPATH"}
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=tmp_path, env=env, timeout=120)
-    assert r.returncode == 0, r.stderr[-2000:]
-    assert np.allclose(np.load(tmp_path / "y.npy"), ours(x[0], update=False))
-    theirs = pickle.load(open(p2, "rb"))["running_state"]          # unpickles into this repo's stand-in (same module path)
+    ours_back, ours_names = _classes(pickle.dumps({"running_state": ours}))
+    theirs, their_names = _classes(g["ref_pickle"].tobytes())
+    assert their_names == {("uhc.khrylib.utils.zfilter", "ZFilter"), ("uhc.khrylib.utils.zfilter", "RunningStat")} and ours_names == their_names
+    theirs = theirs["running_state"]                                  # unpickles into this repo's stand-in (same module path)
+    assert _layout(ours_back["running_state"]) == _layout(theirs)
+    assert np.allclose(g["y_ref_from_ours"], ours(x[0], update=False))
     assert type(theirs).__module__ == "uhc.khrylib.utils.zfilter" and theirs.rs._n == 40
     assert np.allclose(theirs.rs._M, x.mean(0)) and np.allclose(theirs.rs._S, ((x - x.mean(0)) ** 2).sum(0))
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "scripts", "train_uhc.py")), reason="no reference checkout on this machine")
-def test_reference_train_script_file_reaches_the_agent_on_this_package(tmp_path):
-    """The reference's OWN scripts/train_uhc.py, unmodified, executed with cwd = a tree holding this repo's `uhc` package and config layout
-    (train_uhc.py:24 puts the cwd on sys.path).  Without a GPU the run must get through argument parsing, Config, the wandb / flags /
-    agent_dict imports and torch.set_default_dtype(float64) and stop exactly where AgentCopycat asks for a CUDA device -- i.e. the whole
-    import surface of the script resolves against this package.  (With a GPU the same file trains: tests/test_gpu_dropin.py.)"""
+def test_reference_train_script_file_reaches_the_agent_on_this_package(tmp_path, golden_dir):
+    """What the reference's OWN scripts/train_uhc.py and scripts/eval_uhc.py import from `uhc` (tests/golden/reference_script_imports.json, recorded by
+    running the unmodified script files against this package, tools/make_golden.py compat) resolves against a tree holding this repo's `uhc`
+    package and config layout, put on sys.path as the scripts do (train_uhc.py:24 appends the cwd).  Without a GPU the script's sequence
+    -- Config by id from the cwd, torch.set_default_dtype(float64), agent_dict[cfg.agent_name] -- must stop exactly where AgentCopycat asks for
+    a CUDA device.  (With a GPU the same sequence trains: tests/test_gpu_dropin.py.)"""
     import yaml
     from tests.helpers import write_synthetic_pkl
     for d in ("uhc", "uhc_b200", "mujoco_py", "assets"):
@@ -78,8 +80,23 @@ def test_reference_train_script_file_reaches_the_agent_on_this_package(tmp_path)
     base.update(policy_hsize=[64], value_hsize=[64], min_batch_size=256, num_optim_epoch=1, num_envs=8, num_epoch=1)
     base["data_specs"]["file_path"] = write_synthetic_pkl(str(tmp_path / "sample_data" / "clips.pkl"))
     yaml.safe_dump(base, open(tmp_path / "config" / "refscript.yml", "w"))
-    env = dict({k: v for k, v in os.environ.items() if k != "PYTHONPATH"}, WANDB_MODE="disabled", CUDA_VISIBLE_DEVICES="")
-    r = subprocess.run([sys.executable, os.path.join(REF, "scripts", "train_uhc.py"), "--cfg", "refscript", "--no_log"], cwd=tmp_path, env=env,
-                       capture_output=True, text=True, timeout=600)
-    assert "Using: cpu" in r.stdout, (r.stdout[-1500:], r.stderr[-1500:])
+    code = f"""
+import importlib, json, os, sys
+sys.path.append(os.getcwd())
+for script, imports in json.load(open({os.path.join(golden_dir, "reference_script_imports.json")!r})).items():
+    for module, names in imports:
+        m = importlib.import_module(module)
+        assert m.__file__.startswith(os.getcwd()), m.__file__
+        for n in names:
+            assert hasattr(m, n), (script, module, n)
+import torch
+from uhc.utils.config_utils.copycat_config import Config
+from uhc.agents import agent_dict
+cfg = Config(cfg_id="refscript", create_dirs=True)
+assert cfg.get("num_envs") == 8 and os.path.isdir("results/motion_im/refscript/models")
+torch.set_default_dtype(torch.float64)
+agent_dict[cfg.agent_name](cfg, torch.float64, torch.device("cpu"), training=True, checkpoint_epoch=0)
+"""
+    env = dict({k: v for k, v in os.environ.items() if k != "PYTHONPATH"}, CUDA_VISIBLE_DEVICES="")
+    r = subprocess.run([sys.executable, "-c", code], cwd=tmp_path, env=env, capture_output=True, text=True, timeout=600)
     assert r.returncode != 0 and "needs a CUDA device" in r.stderr, r.stderr[-3000:]

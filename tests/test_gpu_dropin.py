@@ -101,16 +101,15 @@ def test_single_env_facade_matches_engine_and_oracle(tmp_path, monkeypatch, gold
     assert np.abs(env.get_humanoid_qpos() - env.get_expert_qpos()).max() < 1e-6
 
 
-def test_reference_script_files_run_against_this_package(tmp_path):
-    """When a checkout of the reference is available ($UHC_REFERENCE, default /root/reference) its OWN script files are executed
-    (scripts/train_uhc.py, then scripts/eval_uhc.py --mode stats) with cwd = a scratch copy of this repo's config/assets layout, so that
-    `sys.path.append(os.getcwd())` (train_uhc.py:24) resolves `uhc` to this package.  Skipped where the reference is absent (the GPU box)."""
+def test_reference_script_files_run_against_this_package(tmp_path, golden_dir):
+    """The reference's scripts/train_uhc.py, then scripts/eval_uhc.py --mode stats, as they run with cwd = a scratch copy of this repo's
+    config/assets layout (`sys.path.append(os.getcwd())`, train_uhc.py:24, resolves `uhc` to this package): every name they import from `uhc`
+    (tests/golden/reference_script_imports.json, recorded from the unmodified script files, tools/make_golden.py compat) resolves there, Config finds
+    the yaml by id under the cwd, training writes the epoch-2 checkpoint under results/ and the evaluation (on the device the eval script passes,
+    the CPU one, eval_uhc.py:84-90) resumes from it."""
     import subprocess
     import sys
     import yaml
-    ref = os.environ.get("UHC_REFERENCE", "/root/reference")
-    if not os.path.exists(os.path.join(ref, "scripts", "train_uhc.py")):
-        pytest.skip("no reference checkout on this machine")
     root = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
     for d in ("uhc", "uhc_b200", "mujoco_py", "assets"):
         if os.path.exists(os.path.join(root, d)):
@@ -121,11 +120,43 @@ def test_reference_script_files_run_against_this_package(tmp_path):
     base["data_specs"]["file_path"] = write_synthetic_pkl(str(tmp_path / "sample_data" / "clips.pkl"))
     base["data_specs"]["t_max"] = 40
     yaml.safe_dump(base, open(tmp_path / "config" / "refscript.yml", "w"))
-    env = dict(os.environ, PYTHONPATH=str(tmp_path), WANDB_MODE="disabled")
-    r = subprocess.run([sys.executable, os.path.join(ref, "scripts", "train_uhc.py"), "--cfg", "refscript", "--no_log"], cwd=tmp_path, env=env,
-                       capture_output=True, text=True, timeout=900)
+    args = dict(cfg="refscript", test=False, num_threads=30, gpu_index=0, show_noise=False, resume=None, no_log=True, debug=False)
+    code = f"""
+import importlib, json, os, sys, types
+sys.path.append(os.getcwd())
+for script, imports in json.load(open({os.path.join(golden_dir, "reference_script_imports.json")!r})).items():
+    for module, names in imports:
+        m = importlib.import_module(module)
+        assert m.__file__.startswith(os.getcwd()), m.__file__
+        for n in names:
+            assert hasattr(m, n), (script, module, n)
+import numpy as np, torch
+from uhc.utils.flags import flags
+from uhc.utils.config_utils.copycat_config import Config
+from uhc.agents import agent_dict
+from uhc.agents.agent_copycat import AgentCopycat
+cfg = Config(cfg_id="refscript", create_dirs=True)
+cfg.update(types.SimpleNamespace(render=False, epoch=0, full_eval=False, **{args!r}))
+flags.debug = False
+torch.set_default_dtype(torch.float64)
+torch.cuda.set_device(0)
+np.random.seed(cfg.seed); torch.manual_seed(cfg.seed)
+agent = agent_dict[cfg.agent_name](cfg, torch.float64, torch.device("cuda", index=0), training=True, checkpoint_epoch=0)
+for i_iter in range(0, cfg.num_epoch):
+    agent.optimize_policy(i_iter)
+    torch.cuda.empty_cache()
+print("training done!")
+cfg = Config(cfg_id="refscript", create_dirs=False)
+cfg.update(types.SimpleNamespace(epoch=2, data={str(tmp_path / "sample_data" / "clips.pkl")!r}, mode="stats", render=False, **{args!r}))
+cfg.no_log = True
+cfg.output = os.path.join("results/renderings/uhc/", cfg.id)
+os.makedirs(cfg.output, exist_ok=True)
+cfg.data_specs["file_path"] = cfg.data
+cfg.data_specs.pop("test_file_path", None)
+np.random.seed(cfg.seed); torch.manual_seed(cfg.seed)
+AgentCopycat(cfg, torch.float64, torch.device("cpu"), training=True, checkpoint_epoch=2).eval_policy(epoch=2, dump=True)
+"""
+    env = {k: v for k, v in os.environ.items() if k != "PYTHONPATH"}
+    r = subprocess.run([sys.executable, "-c", code], cwd=tmp_path, env=env, capture_output=True, text=True, timeout=900)
     assert r.returncode == 0 and "training done!" in r.stdout, r.stderr[-3000:]
     assert os.path.exists(tmp_path / "results" / "motion_im" / "refscript" / "models" / "iter_0002.p")
-    r = subprocess.run([sys.executable, os.path.join(ref, "scripts", "eval_uhc.py"), "--cfg", "refscript", "--epoch", "2", "--mode", "stats"], cwd=tmp_path,
-                       env=env, capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, r.stderr[-3000:]

@@ -389,8 +389,75 @@ def gen_math():
     print("math goldens ok", out["mul_doctest"])
 
 
+# the configuration keys uhc.agents.agent_copycat.supported_variant reads, and the one the drop-in dispatches on
+SUPPORTED_VARIANT_KEYS = ("agent_name", "obs_v", "actor_type", "reward_id", "fix_std", "residual_force", "obs_vel", "obs_coord", "obs_phase", "has_shape",
+                         "env_term_body", "residual_force_mode", "residual_force_bodies", "residual_force_torque", "residual_force_bodies_num",
+                         "residual_contact_only", "residual_contact_projection", "env_init_noise")
+
+
+def gen_compat():
+    """The drop-in boundary, recorded from the reference's own code for tests/test_checkpoint_compat.py, tests/test_shim_cpu.py and
+    tests/test_gpu_dropin.py:
+      reference_configs.json        the keys supported_variant reads, of every yaml under the reference's config/
+      zfilter_roundtrip.npz         a running_state pickled by the reference's ZFilter (40 rows of x ~ RandomState(1).normal(0.5, 3, (40, 657))
+                                    pushed one by one), and the reference's ZFilter applied to x[0] after loading this repo's pickle of the same statistics
+      reference_script_imports.json what scripts/train_uhc.py and scripts/eval_uhc.py import from `uhc` / `mujoco_py` when they run with this
+                                    repo's package on a machine without a CUDA device (they stop where AgentCopycat asks for one)"""
+    import glob
+    import json
+    import shutil
+    import subprocess
+    import tempfile
+    import yaml
+    views = {}
+    for f in sorted(glob.glob(os.path.join(H.REF, "config", "**", "*.yml"), recursive=True)):
+        d = yaml.safe_load(open(f)) or {}
+        views[os.path.relpath(f, os.path.join(H.REF, "config"))] = {k: d[k] for k in SUPPORTED_VARIANT_KEYS if k in d}
+    json.dump(views, open(os.path.join(OUT, "reference_configs.json"), "w"), indent=0, sort_keys=True)
+
+    work = tempfile.mkdtemp(prefix="uhc_compat_")
+    env = {k: v for k, v in os.environ.items() if k != "PYTHONPATH"}
+    run = lambda code, path, cwd=work, **kw: subprocess.run([sys.executable, "-c", f"import sys; sys.path.insert(0, {path!r})\n" + code], cwd=cwd,
+                                                           env=dict(env, **kw), check=True)
+    xs = "import numpy as np, pickle\nx = np.random.RandomState(1).normal(0.5, 3.0, (40, 657))\n"
+    run(xs + "from uhc.khrylib.utils.zfilter import ZFilter\n"
+        "pickle.dump({'running_state': ZFilter.from_stats(40, x.mean(0), ((x - x.mean(0)) ** 2).sum(0), clip=5.0)}, open('ours.p', 'wb'))", H.ROOT)
+    run(xs + f"from uhc.khrylib.utils import zfilter\nassert zfilter.__file__.startswith({H.REF!r})\n"
+        "np.save('y.npy', pickle.load(open('ours.p', 'rb'))['running_state'](x[0], update=False))\n"
+        "z = zfilter.ZFilter((657,), clip=5)\nfor r in x: z(r)\npickle.dump({'running_state': z}, open('ref.p', 'wb'))", H.REF)
+    np.savez_compressed(os.path.join(OUT, "zfilter_roundtrip.npz"), y_ref_from_ours=np.load(os.path.join(work, "y.npy")),
+                        ref_pickle=np.frombuffer(open(os.path.join(work, "ref.p"), "rb").read(), np.uint8))
+
+    sys.path.insert(0, H.ROOT)
+    from tests.helpers import write_synthetic_pkl
+    for d in ("uhc", "uhc_b200", "mujoco_py"):
+        os.symlink(os.path.join(H.ROOT, d), os.path.join(work, d))
+    os.makedirs(os.path.join(work, "config"))
+    base = yaml.safe_load(open(os.path.join(H.ROOT, "config", "uhc_b200_default.yml")))
+    base["data_specs"]["file_path"] = write_synthetic_pkl(os.path.join(work, "sample_data", "clips.pkl"))
+    yaml.safe_dump(base, open(os.path.join(work, "config", "refscript.yml"), "w"))
+    imports = {}
+    for script, argv in (("train_uhc.py", ["--cfg", "refscript", "--no_log"]), ("eval_uhc.py", ["--cfg", "refscript", "--epoch", "2", "--mode", "stats"])):
+        path = os.path.join(H.REF, "scripts", script)
+        code = (f"import builtins, json, runpy\nrec, imp = [], builtins.__import__\n"
+                "def hook(name, g=None, l=None, fromlist=(), level=0):\n"
+                f"    if (g or {{}}).get('__file__') == {path!r} and name.split('.')[0] in ('uhc', 'mujoco_py'):\n"
+                "        rec.append([name, sorted(fromlist or ())])\n"
+                "    return imp(name, g, l, fromlist, level)\n"
+                f"builtins.__import__ = hook\nsys.argv = [{path!r}] + {argv!r}\n"
+                f"try:\n    runpy.run_path({path!r}, run_name='__main__')\nexcept RuntimeError as e:\n    assert 'needs a CUDA device' in str(e), e\n"
+                "json.dump(rec, open('imports.json', 'w'))")
+        run(code, work, WANDB_MODE="disabled", CUDA_VISIBLE_DEVICES="")
+        imports["scripts/" + script] = json.load(open(os.path.join(work, "imports.json")))
+    json.dump(imports, open(os.path.join(OUT, "reference_script_imports.json"), "w"), indent=1)
+    shutil.rmtree(work)
+    print("compat goldens:", len(views), "configs;", imports)
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
+    if sys.argv[1:] == ["compat"]:            # needs the reference checkout, not the harness's stubs
+        return gen_compat()
     H.install()
     what = sys.argv[1:] or ["math", "env", "ppo"]
     if "math" in what:
