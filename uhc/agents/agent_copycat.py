@@ -4,7 +4,7 @@
   .optimize_policy(epoch)   per_epoch_update -> sample -> update_params -> checkpoint / eval every save_n_epochs -> log   (:326-352)
   .sample(min_batch_size)   -> (batch, log)      batch: states / actions / masks / rewards / exps (device resident, numpy on demand)
   .update_params(batch)     GAE + PPO epochs (khrylib agent_pg.py:39-56, agent_ppo.py:16-51)
-  .eval_policy(epoch, dump) deterministic roll-out of every clip, coverage / error statistics                               (:354-494)
+  .eval_policy(epoch, dump) deterministic roll-out of every clip on the device (uhc_evaluate), coverage / error statistics (:354-494)
   .save_checkpoint / .load_checkpoint   pickle {"policy_dict", "value_dict", "running_state"} at models/iter_%04d.p        (:190-260)
 
 Differences that are inherent to the batched design are listed in DESIGN.md (lock-step horizon with value bootstrap, batched
@@ -24,7 +24,6 @@ import numpy as np
 from uhc.data_loaders.dataset_amass_single import DatasetAMASSSingle
 from uhc.envs.humanoid_im import HumanoidEnv
 from uhc.losses.reward_function import reward_func
-from uhc_b200 import nn
 from uhc_b200.agent import BatchedAgent, RolloutBuffer, make_nccl_grad_sync
 from uhc_b200.model import HumanoidModel
 
@@ -195,74 +194,39 @@ class AgentCopycat:
             except Exception:
                 pass
 
-    # ---------------------------------------------------------------- evaluation (:354-494), batched: one env per clip
+    # ---------------------------------------------------------------- evaluation (:354-494) on the device: BatchedAgent.evaluate
     def eval_policy(self, epoch=0, dump=False):
-        """eval_policy / eval_seq (agent_copycat.py:354-494) for every clip at once: env i imitates clip c0 + i from frame 0 with the
-        deterministic policy; per step ONE batched state read (uhc_env_get_state_batch) feeds the reference's metrics
-        (smpl_eval.compute_metrics: mpjpe / pa-mpjpe / accel / vel / root distance, restated in uhc_b200/metrics.py); fail_safe re-seats a
-        failed humanoid on the expert pose with one batched set_state (humanoid_im.py:902-905)."""
-        import torch
-        from uhc_b200.metrics import compute_metrics
+        """eval_policy / eval_seq (agent_copycat.py:354-494) for every clip: each clip is imitated from frame 0 with the deterministic policy
+        (uhc_evaluate: a work queue of clips over the env slots, fail_safe re-seating a failed humanoid on the expert pose inside the step
+        kernel, humanoid_im.py:902-905), and scored on the device with the reference's metrics (smpl_eval.compute_metrics: mpjpe / pa-mpjpe /
+        accel / vel / root distance, restated in uhc_b200/metrics.py)."""
+        from uhc_b200.agent import EVAL_METRICS
         cfg = self.cfg
         res_dicts = []
         eng = self.agent.engine
-        E = self.num_envs
         for loader in self.test_data_loaders:
             n = loader.get_len()
             if loader is not self.data_loader:
-                eng.load_clips(loader.experts, loader.shapes)      # invalidates every env record: only the envs reset below are stepped
+                eng.load_clips(loader.experts, loader.shapes)      # invalidates every env record: evaluate resets the slots it runs
             eng.set_cfg(**self._env_cfg(test=True))
+            ev = self.agent.evaluate(0, n, bool(cfg.fail_safe))
             res = {}
-            for c0 in range(0, n, E):
-                ids = np.arange(min(E, n - c0), dtype=np.int32)
-                clips = (c0 + ids).astype(np.int32)
-                if len(ids) < E:                                   # idle envs: park them on clip c0 so every record is valid (their outputs are ignored)
-                    eng.reset(np.arange(len(ids), E, dtype=np.int32), np.full(E - len(ids), c0, np.int32), 0, None)
-                obs = eng.reset(ids, clips, 0, None)
-                lens = eng.clip_len[clips]
-                alive = np.ones(len(ids), bool); fail_any = np.zeros(len(ids), bool)
-                rsum = np.zeros(len(ids)); last_t = np.zeros(len(ids), np.int64)
-                traj = [dict(pred=[], pred_jpos=[], t=[]) for _ in ids]
-                det = torch.ones(E, dtype=torch.uint8, device=obs.device)
-                for t in range(int(lens.max()) - 1):
-                    s = self.running_state(obs, update=False)
-                    mean = self.policy_net.forward_tc(s)
-                    a, _ = nn.gaussian_sample(mean, self.agent.log_std, 0, 0, det)
-                    obs, rew, ci, fail, end, pct = eng.step(a)
-                    f, e, r = fail.cpu().numpy()[ids] != 0, end.cpu().numpy()[ids] != 0, rew.cpu().numpy()[ids]
-                    live = np.nonzero(alive)[0]
-                    st = eng.get_states(ids[live])
-                    for j, i in enumerate(live):
-                        traj[i]["pred"].append(st["qpos"][j].copy()); traj[i]["pred_jpos"].append(st["xpos"][j].reshape(-1).copy()); traj[i]["t"].append(int(st["cur_t"][j]))
-                        last_t[i] = st["cur_t"][j]
-                    rsum[live] += r[live]
-                    failed = live[f[live]]
-                    fail_any[failed] = True
-                    if len(failed):
-                        if cfg.fail_safe:
-                            tt = [min(int(last_t[i]), loader.experts[clips[i]]["len"] - 1) for i in failed]
-                            eng.set_states(ids[failed], np.stack([loader.experts[clips[i]]["qpos"][k] for i, k in zip(failed, tt)]),
-                                           np.stack([loader.experts[clips[i]]["qvel"][k] for i, k in zip(failed, tt)]))
-                        else:
-                            alive[failed] = False
-                    alive[live[e[live]]] = False
-                    if not alive.any():
-                        break
-                for i in ids:
-                    k = loader.data_keys[c0 + i]
-                    ex = loader.experts[clips[i]]
-                    tt = np.minimum(np.array(traj[i]["t"], dtype=np.int64), ex["len"] - 1)
-                    percent = float(last_t[i]) / float(max(lens[i] - 1, 1))
-                    r_i = {"pred": np.array(traj[i]["pred"]), "gt": np.asarray(ex["qpos"])[tt], "pred_jpos": np.array(traj[i]["pred_jpos"]),
-                           "gt_jpos": np.asarray(ex["wbpos"])[tt], "percent": 1.0 if (percent >= 1.0 and not fail_any[i]) else min(percent, 0.999),
-                           "fail_safe": bool(fail_any[i] and cfg.fail_safe)}
-                    m = compute_metrics(r_i) if len(tt) >= 3 else {"succ": np.array([False])}
-                    m["succ"] = np.array([bool(m["succ"][0]) and not fail_any[i]])
-                    m["reward"] = rsum[i] / max(lens[i] - 1, 1)
-                    m["percent"] = percent
-                    res[k] = m
-                    if k in self.freq_dict:      # eval outcome feeds the failure-weighted sampler like a training episode ([percent, fr_start])
-                        self.freq_dict[k] = (self.freq_dict[k] + [[1.0 if m["succ"][0] else min(percent, 0.999), 0]])[-self.max_freq:]
+            for i in range(n):
+                k = loader.data_keys[i]
+                L, fail_any = int(eng.clip_len[i]), bool(ev["fail_any"][i])
+                percent = float(ev["last_t"][i]) / float(max(L - 1, 1))
+                if ev["nframes"][i] >= 3:
+                    fm = dict(zip(EVAL_METRICS, ev["frame_metrics"][i].T))
+                    m = {"root_dist": fm["root_dist"], "mpjpe_g": fm["mpjpe_g"], "pa_mpjpe": fm["pa_mpjpe"], "mpjpe": fm["mpjpe"],
+                         "accel_dist": fm["accel_dist"][2:], "vel_dist": fm["vel_dist"][1:]}
+                    m["succ"] = np.array([percent >= 1.0 and not fail_any])
+                else:
+                    m = {"succ": np.array([False])}
+                m["reward"] = ev["reward_sum"][i] / max(L - 1, 1)
+                m["percent"] = percent
+                res[k] = m
+                if k in self.freq_dict:      # eval outcome feeds the failure-weighted sampler like a training episode ([percent, fr_start])
+                    self.freq_dict[k] = (self.freq_dict[k] + [[1.0 if m["succ"][0] else min(percent, 0.999), 0]])[-self.max_freq:]
             if loader is not self.data_loader:
                 eng.load_clips(self.data_loader.experts, self.data_loader.shapes)
             eng.set_cfg(**self._env_cfg(test=False))

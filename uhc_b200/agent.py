@@ -24,6 +24,15 @@ class UhcRolloutBuf(C.Structure):
                [("T_cap", C.c_int), ("reserved", C.c_int)]
 
 
+class UhcEvalBuf(C.Structure):
+    """include/uhc_eval.h UhcEvalBuf"""
+    _fields_ = [(k, C.c_void_p) for k in ("frame_off", "pred_qpos", "pred_jpos", "frame_t", "frame_metrics", "nframes", "last_t", "fail_any", "reward_sum",
+                                         "clip_metrics")] + [("frame_cap", C.c_int), ("reserved", C.c_int)]
+
+
+EVAL_METRICS = ("root_dist", "mpjpe", "mpjpe_g", "pa_mpjpe", "vel_dist", "accel_dist")      # frame_metrics / clip_metrics columns
+
+
 def ewma(x, alpha=0.05):
     """uhc/utils/math_utils.py:25-29"""
     avg = float(x[0])
@@ -184,8 +193,7 @@ class BatchedAgent:
             L.uhc_rollout_last_error.restype = C.c_char_p
             self._ro_ready = True
         mcp = self.actor_type == "mcp"
-        if self.policy._bf16 is None or getattr(self, "_mlp_c", None) is None:
-            self._mlp_c = nn.mcp_struct(self.policy) if mcp else nn.mlp_struct(self.policy)
+        self._policy_struct()
         if getattr(self, "_ro_step", None) != self.global_step:
             L.uhc_rollout_set_step(self.engine.h, C.c_ulonglong(self.global_step))
         bs = buf.c_struct(self.obs)
@@ -198,6 +206,53 @@ class BatchedAgent:
         self.global_step += T
         self._ro_step = self.global_step
         self.nn_launches += T * (L.uhc_rollout_launches_per_step(self.engine.h) - 1)      # the env-step launch is counted by the engine
+
+    def _policy_struct(self):
+        if self.policy._bf16 is None or getattr(self, "_mlp_c", None) is None:
+            self._mlp_c = nn.mcp_struct(self.policy) if self.actor_type == "mcp" else nn.mlp_struct(self.policy)
+        return self._mlp_c
+
+    def evaluate(self, clip0, n, fail_safe, trajectories=False):
+        """Deterministic evaluation of clips [clip0, clip0 + n) of the loaded table from frame 0 (uhc_evaluate, include/uhc_eval.h): a device
+        work queue of clips over the env slots, fail_safe re-seating inside the step kernel, metrics on the device.  Uses the env records (the
+        next sample() must reset them: set self.obs = None).  Returns numpy arrays per clip: nframes, last_t, fail_any, reward_sum,
+        clip_metrics [n][6] (columns EVAL_METRICS, mm), frame_metrics (list of [nframes][6]), steps (control steps run); with trajectories
+        also pred_qpos / pred_jpos / frame_t (lists of [nframes][...])."""
+        t = self.torch
+        L = self.engine.lib
+        if not getattr(self, "_ev_ready", False):
+            L.uhc_eval_last_error.restype = C.c_char_p
+            self._ev_ready = True
+        clip0, n = int(clip0), int(n)
+        lens = np.asarray(self.engine.clip_len[max(clip0, 0):max(clip0 + n, 0)], np.int64)
+        rows = np.maximum(lens - 1 + max(int(self.engine._cfg.trail_steps), 0), 0)
+        off = np.zeros(max(n, 0) + 1, np.int32)
+        off[1:len(rows) + 1] = np.cumsum(rows)
+        off[len(rows) + 1:] = off[len(rows)]
+        F, nn_ = max(int(off[-1]), 1), max(n, 1)
+        d, i32, f64 = self.dev, t.int32, t.float64
+        o = dict(frame_off=t.as_tensor(off, device=d), pred_qpos=t.empty(F, 76, device=d, dtype=t.float32), pred_jpos=t.empty(F, 72, device=d, dtype=t.float32), frame_t=t.empty(F, device=d, dtype=i32),
+                 frame_metrics=t.empty(F, 6, device=d, dtype=f64), nframes=t.empty(nn_, device=d, dtype=i32), last_t=t.empty(nn_, device=d, dtype=i32),
+                 fail_any=t.empty(nn_, device=d, dtype=i32), reward_sum=t.empty(nn_, device=d, dtype=f64), clip_metrics=t.empty(nn_, 6, device=d, dtype=f64))
+        b = UhcEvalBuf()
+        for k, v in o.items():
+            setattr(b, k, v.data_ptr())
+        b.frame_cap = int(off[-1])
+        st = C.c_void_p(t.cuda.current_stream(self.dev).cuda_stream)
+        fn = L.uhc_evaluate_mcp if self.actor_type == "mcp" else L.uhc_evaluate
+        rc = fn(self.engine.h, C.c_int(clip0), C.c_int(n), C.byref(self._policy_struct()), C.c_void_p(self.log_std.data_ptr()),
+                C.c_void_p(self.running_state.stats.data_ptr()), C.c_float(self.running_state.clip), C.c_int(int(bool(fail_safe))), C.byref(b), st)
+        if rc != 0:
+            raise RuntimeError("uhc_evaluate: " + L.uhc_eval_last_error().decode())
+        steps = C.c_longlong(0)
+        L.uhc_eval_last_steps(self.engine.h, C.byref(steps))
+        h = {k: v.cpu().numpy() for k, v in o.items() if trajectories or k not in ("pred_qpos", "pred_jpos", "frame_t")}
+        nf = h["nframes"][:n]
+        out = dict(nframes=nf, last_t=h["last_t"][:n], fail_any=h["fail_any"][:n] != 0, reward_sum=h["reward_sum"][:n], clip_metrics=h["clip_metrics"][:n],
+                   steps=int(steps.value))
+        for k in ("frame_metrics",) + (("pred_qpos", "pred_jpos", "frame_t") if trajectories else ()):
+            out[k] = [h[k][off[i]:off[i] + nf[i]] for i in range(n)]
+        return out
 
     def sample(self, T, buf=None, use_tc=True, c_loop=None):
         """agent.sample(): T lock-step control steps of all envs.  Returns (buffer, log).  c_loop (default: whenever auto_reset is on):

@@ -4,8 +4,8 @@ import subprocess
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SO = os.path.join(HERE, "libuhc_b200.so")
-SRCS = ["step_kernel.cu", "nn_kernels.cu", "mlp_tcgen05.cu", "rollout.cu", "ppo_update.cu"]
-DEPS = ["sim_core.h", "env_step.h", "../../include/uhc_b200.h", "../../include/uhc_nn.h", "../../include/uhc_rollout.h", "../../include/uhc_ppo.h"]
+SRCS = ["step_kernel.cu", "nn_kernels.cu", "mlp_tcgen05.cu", "rollout.cu", "ppo_update.cu", "eval.cu"]
+DEPS = ["sim_core.h", "env_step.h", "eval_internal.h", "eval_metrics.h", "../../include/uhc_b200.h", "../../include/uhc_nn.h", "../../include/uhc_rollout.h", "../../include/uhc_ppo.h", "../../include/uhc_eval.h"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "--use_fast_math=false",
               "-Xcompiler", "-fPIC", "-shared", "-Xptxas", "-v", "--expt-relaxed-constexpr"]
 

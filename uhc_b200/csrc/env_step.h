@@ -26,6 +26,21 @@ struct EngineView {
     int *counters;          // [4] device counters: 0 = env-steps failed because a body's contacts did not fit MAXCON, 1 = env-steps skipped on an invalid env record
 };
 
+// evaluation mode of the step kernel (uhc_evaluate, eval.cu): a work queue of clips [clip0, clip0 + n) over the env slots.  Slot e
+// imitates clip clip0 + slot_clip[e] from frame 0 (-1: idle, no physics); every step of an active slot is recorded into row
+// frame_off[i] + slot_k[e] of the per-frame outputs; a finished slot takes the next clip from queue[0] or goes idle (queue[1] counts the
+// active slots).
+struct EvalView {
+    int clip0, n, fail_safe, reserved;
+    const int *frame_off;           // [n+1]
+    float *pred_qpos, *pred_jpos;   // [F][76], [F][72]
+    int *frame_t;                   // [F]
+    int *nframes, *last_t, *fail_any;   // [n]
+    double *reward_sum;             // [n]
+    int *slot_clip, *slot_k;        // [E]
+    int *queue;                     // [2]
+};
+
 // an env record the step kernel can run: a clip of the CURRENT clip table and at least two frames (uhc_load_clips invalidates every
 // record; never-reset envs have len = 0)
 template <class Real>
@@ -164,7 +179,9 @@ UHC_DEV void store_state(const EngineView<Real> &ev, int env, Work<Real> &w) {
 
 // reset one env onto frame 0 of (clip, start, len): state <- expert qpos/qvel (or the override), sim.forward(), obs.
 // bquat is left at the qpos0 value (identity quats) exactly as reset_model leaves it (humanoid_im.py:1277 runs before set_state).
-template <class Real, class ObsT>
+// RESEAT: the fail-safe re-seat of uhc_env_set_state_batch (humanoid_im.py:902-905): qpos / qvel overridden, cur_t and the body
+// quaternions (bquat, prev_bquat) of the running episode kept
+template <class Real, class ObsT, bool RESEAT = false>
 UHC_DEV void env_reset_warp(const EngineView<Real> &ev, int env, Work<Real> &w, int clip, int start, int len,
                             const Real *qpos_override, const Real *qvel_override, ObsT *obs) {
     const Real *e0 = expert_frame(ev, clip, start, len, 0);
@@ -199,8 +216,8 @@ UHC_DEV void env_reset_warp(const EngineView<Real> &ev, int env, Work<Real> &w, 
     int *is = ev.istate + (size_t)env * SI_SIZE;
     Real *st = ev.state + (size_t)env * ST_SIZE;
     LANES_BEGIN
-    for (int i = lane; i < 96; i += 32) { const Real v = (i & 3) == 0 ? Real(1) : Real(0); st[ST_BQUAT + i] = v; st[ST_PBQUAT + i] = v; }
-    if (lane == 0) { is[SI_CUR_T] = 0; is[SI_CLIP] = clip; is[SI_START] = start; is[SI_LEN] = len; is[SI_NEWTON] = iters; is[SI_NCON] = w.ncon; }
+    if constexpr (!RESEAT) for (int i = lane; i < 96; i += 32) { const Real v = (i & 3) == 0 ? Real(1) : Real(0); st[ST_BQUAT + i] = v; st[ST_PBQUAT + i] = v; }
+    if (lane == 0) { if constexpr (!RESEAT) is[SI_CUR_T] = 0; is[SI_CLIP] = clip; is[SI_START] = start; is[SI_LEN] = len; is[SI_NEWTON] = iters; is[SI_NCON] = w.ncon; }
     LANES_END
     if (obs) write_obs(ev, w, clip, start, len, 1, obs);
     LANES_BEGIN
@@ -209,10 +226,70 @@ UHC_DEV void env_reset_warp(const EngineView<Real> &ev, int env, Work<Real> &w, 
     store_state(ev, env, w);
 }
 
-// one control step.  out_* may be null.  Returns done; fills flags.
+// evaluation epilogue of an active slot (EvalView): record the step, then fail-safe re-seat, or hand the slot the next clip of the queue
 template <class Real, class ObsT>
+UHC_DEV void eval_after_step(const EngineView<Real> &ev, const EvalView &xv, int env, Work<Real> &w, int cur_t, int fail, int end, Real rew, ObsT *obs) {
+    int *is = ev.istate + (size_t)env * SI_SIZE;
+    const int i = xv.slot_clip[env], k = xv.slot_k[env];
+    const int row = xv.frame_off[i] + k;
+    if (row < xv.frame_off[i + 1]) {       // the caller's table holds len - 1 + trail_steps rows per clip: always true
+        LANES_BEGIN
+        for (int j = lane; j < NQ; j += 32) xv.pred_qpos[(size_t)row * NQ + j] = (float)w.q[j];
+        for (int j = lane; j < 72; j += 32) xv.pred_jpos[(size_t)row * 72 + j] = (float)(&w.xpos[0][0])[j];     // the stored xpos (get_states)
+        if (lane == 0) {
+            xv.frame_t[row] = cur_t; xv.nframes[i] = k + 1; xv.last_t[i] = cur_t;
+            xv.reward_sum[i] += (double)(ObsT)rew;
+            if (fail) xv.fail_any[i] = 1;
+        }
+        LANES_END
+    }
+    if (!end && !(fail && !xv.fail_safe)) {
+        if (fail) {   // fail_safe: the expert pose at min(cur_t, len - 1), sim.forward(); the step's own observation stays the next input
+            const int clip = is[SI_CLIP], start = is[SI_START], len = is[SI_LEN];
+            const Real *ef = expert_frame(ev, clip, start, len, cur_t);
+            const Real *qo = ef + EX_QPOS, *vo = ef + EX_QVEL;
+            if constexpr (sizeof(Real) != sizeof(float)) {   // uhc_env_set_state_batch passes the pose as float: stage it rounded, as k_env_reset does
+                Real *q = w.as_, *v = w.Mp;
+                LANES_BEGIN
+                for (int j = lane; j < NQ; j += 32) q[j] = (Real)(float)qo[j];
+                for (int j = lane; j < NV; j += 32) v[j] = (Real)(float)vo[j];
+                LANES_END
+                qo = q; vo = v;
+            }
+            env_reset_warp<Real, ObsT, true>(ev, env, w, clip, start, len, qo, vo, (ObsT *)nullptr);
+        }
+        LANES_BEGIN
+        if (lane == 0) xv.slot_k[env] = k + 1;
+        LANES_END
+        return;
+    }
+    int j;      // the episode ended: next clip of the queue, or idle
+#ifndef UHC_EMU
+    j = (threadIdx.x & 31) == 0 ? atomicAdd(xv.queue, 1) : 0;
+    j = __shfl_sync(0xffffffffu, j, 0);
+#else
+    j = xv.queue[0]++;
+#endif
+    if (j < xv.n) {
+        const int c = xv.clip0 + j;
+        env_reset_warp<Real, ObsT>(ev, env, w, c, 0, UHC_LDG(ev.clip_adr + c + 1) - UHC_LDG(ev.clip_adr + c), (const Real *)nullptr, (const Real *)nullptr, obs);
+    }
+    LANES_BEGIN
+    if (lane == 0) {
+        xv.slot_clip[env] = j < xv.n ? j : -1; xv.slot_k[env] = 0;
+#ifndef UHC_EMU
+        if (j >= xv.n) atomicSub(xv.queue + 1, 1);
+#else
+        if (j >= xv.n) xv.queue[1]--;
+#endif
+    }
+    LANES_END
+}
+
+// one control step.  out_* may be null.  Returns done; fills flags.  EVAL: the evaluation epilogue (xv) replaces auto_reset.
+template <class Real, class ObsT, bool EVAL = false>
 UHC_DEV int env_step_warp(const EngineView<Real> &ev, int env, Work<Real> &w, const ObsT *action, ObsT *obs, ObsT *reward,
-                          ObsT *cinfo_out, int *fail_out, int *end_out, ObsT *percent_out, ObsT *torque_out) {
+                          ObsT *cinfo_out, int *fail_out, int *end_out, ObsT *percent_out, ObsT *torque_out, const EvalView *xv = nullptr) {
     int *is = ev.istate + (size_t)env * SI_SIZE;
     Real *st = ev.state + (size_t)env * ST_SIZE;
     const int clip = is[SI_CLIP], start = is[SI_START], len = is[SI_LEN];
@@ -305,6 +382,10 @@ UHC_DEV int env_step_warp(const EngineView<Real> &ev, int env, Work<Real> &w, co
     if (cinfo_out && lane < 5) cinfo_out[lane] = (ObsT)ci[lane];
     LANES_END
     store_state(ev, env, w);
+    if constexpr (EVAL) {
+        eval_after_step<Real, ObsT>(ev, *xv, env, w, cur_t, fail, end, rew, obs);
+        return fail || end;
+    }
     if (ev.cfg.auto_reset && (fail || end)) {   // re-seed the finished episode in place: the next observation is the reset observation
         int nclip, nstart, nlen;
         const int episode = is[SI_EPISODE] + 1;

@@ -11,6 +11,7 @@
 #define UHC_EPB_F 7
 #endif
 #include "env_step.h"
+#include "eval_internal.h"
 
 using namespace uhc;
 
@@ -40,10 +41,14 @@ __device__ __forceinline__ void stage_tables(EngineView<Real> &ev, unsigned char
 #else
 #define UHC_STEP_BOUNDS(EPB, Real) __launch_bounds__(32 * EPB, (sizeof(Real) == 4 && EPB <= 7 ? UHC_MIN_CTAS : 1))
 #endif
-template <class Real, int EPB>
+// EVAL: the evaluation mode of uhc_evaluate (EvalView, env_step.h): idle slots return at once (no physics, not counted as invalid),
+// active slots record their step and take the next clip of the queue in place of auto_reset.  The rollout instantiation (EVAL = false)
+// never reads xv.
+template <class Real, int EPB, bool EVAL = false>
 __global__ void UHC_STEP_BOUNDS(EPB, Real)
 k_env_step(EngineView<Real> ev, const float *__restrict__ act, float *__restrict__ obs, float *__restrict__ rew, float *__restrict__ cinfo,
-           int *__restrict__ fail, int *__restrict__ end, float *__restrict__ pct, float *__restrict__ torque, const int *__restrict__ order) {
+           int *__restrict__ fail, int *__restrict__ end, float *__restrict__ pct, float *__restrict__ torque, const int *__restrict__ order,
+           const __grid_constant__ EvalView xv) {
     extern __shared__ __align__(16) unsigned char smem[];
 #ifndef UHC_SYNC_SPLIT
 #define UHC_SYNC_SPLIT EPB            /* warps per alignment group (experiment knob; measured: the whole CTA is best) */
@@ -55,20 +60,21 @@ k_env_step(EngineView<Real> ev, const float *__restrict__ act, float *__restrict
     // the warps of a CTA wait for each other every substep: `order` groups environments that needed a similar number of solver
     // iterations in the previous step into the same CTA (k_order_envs), outputs stay indexed by the environment id
     const int env = slot < ev.num_envs ? (order ? order[slot] : slot) : -1;
-    const bool valid = env >= 0 && env_record_valid(ev, env);
+    const bool idle = EVAL && env >= 0 && xv.slot_clip[env] < 0;
+    const bool valid = env >= 0 && !idle && env_record_valid(ev, env);
     if (valid && (threadIdx.x & 31) == 0) atomicAdd(&s_nvalid[grp], 1);
     __syncthreads();
     if (!valid) {   // no work (grid tail) or a stale / never-reset env record: flagged outputs, and the warp is not counted in the substep barrier
-        if (env >= 0) env_step_invalid<Real, float>(ev, obs ? obs + (size_t)env * ev.cfg.obs_dim : nullptr, rew ? rew + env : nullptr, cinfo ? cinfo + (size_t)env * 5 : nullptr,
+        if (env >= 0 && !idle) env_step_invalid<Real, float>(ev, obs ? obs + (size_t)env * ev.cfg.obs_dim : nullptr, rew ? rew + env : nullptr, cinfo ? cinfo + (size_t)env * 5 : nullptr,
                                                     fail ? fail + env : nullptr, end ? end + env : nullptr, pct ? pct + env : nullptr);
         return;
     }
     Work<Real> &w = reinterpret_cast<Work<Real> *>(smem)[warp];
     if ((threadIdx.x & 31) == 0) { w.sync_threads = 32 * s_nvalid[grp]; w.sync_id = 1 + grp; }
     state_mbar_init(w);            // mbarrier of this warp's bulk-async (TMA) state load
-    env_step_warp<Real, float>(ev, env, w, act + (size_t)env * ev.cfg.act_dim, obs ? obs + (size_t)env * ev.cfg.obs_dim : nullptr, rew ? rew + env : nullptr,
-                               cinfo ? cinfo + (size_t)env * 5 : nullptr, fail ? fail + env : nullptr, end ? end + env : nullptr,
-                               pct ? pct + env : nullptr, torque ? torque + (size_t)env * NSUB * NU : nullptr);
+    env_step_warp<Real, float, EVAL>(ev, env, w, act + (size_t)env * ev.cfg.act_dim, obs ? obs + (size_t)env * ev.cfg.obs_dim : nullptr, rew ? rew + env : nullptr,
+                                     cinfo ? cinfo + (size_t)env * 5 : nullptr, fail ? fail + env : nullptr, end ? end + env : nullptr,
+                                     pct ? pct + env : nullptr, torque ? torque + (size_t)env * NSUB * NU : nullptr, &xv);
 }
 
 // counting sort of the environments by the Newton iterations of their previous step (one block)
@@ -227,12 +233,14 @@ int uhc_engine_create(const UhcModelHost *model, const UhcEnvCfg *cfg, int num_e
     }
     if (precision == 32) {
         CK(cudaFuncSetAttribute(k_env_step<float, EPB_F>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)step_smem<float, EPB_F>()));
+        CK(cudaFuncSetAttribute(k_env_step<float, EPB_F, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)step_smem<float, EPB_F>()));
         CK(cudaFuncSetAttribute(k_env_reset<float, EPB_F>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)step_smem<float, EPB_F>()));
         int resident = 0;
         CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, k_env_step<float, EPB_F>, 32 * EPB_F, step_smem<float, EPB_F>()));
         if (EPB_F == 7 && resident < UHC_MIN_CTAS) { g_err = "uhc_engine_create: k_env_step<float> reaches only " + std::to_string(resident) + " resident block(s) per SM (built for " + std::to_string(UHC_MIN_CTAS) + ")"; delete e; return -3; }
     } else {
         CK(cudaFuncSetAttribute(k_env_step<double, EPB_D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)step_smem<double, EPB_D>()));
+        CK(cudaFuncSetAttribute(k_env_step<double, EPB_D, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)step_smem<double, EPB_D>()));
         CK(cudaFuncSetAttribute(k_env_reset<double, EPB_D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)step_smem<double, EPB_D>()));
     }
     const size_t E = num_envs;
@@ -359,8 +367,9 @@ int uhc_set_clip_models(UhcEngine *e, int nclips, const int *clip_model) {
     return 0;
 }
 
-int uhc_env_reset(UhcEngine *e, int n, const int *env_ids_host, const int *clip_host, const int *start_host, const int *len_host,
-                  const float *qpos_dev, const float *qvel_dev, float *obs_dev, void *stream) {
+// no_auto_reset: the launch sees auto_reset = 0 whatever the engine's configuration (evaluation: no reactive standing-neutral starts)
+static int env_reset_impl(UhcEngine *e, int n, const int *env_ids_host, const int *clip_host, const int *start_host, const int *len_host,
+                          const float *qpos_dev, const float *qvel_dev, float *obs_dev, void *stream, bool no_auto_reset) {
     if (!e || n <= 0 || !env_ids_host || !clip_host || !start_host || !len_host) { g_err = "uhc_env_reset: bad argument"; return -2; }
     if (!e->d_expert) { g_err = "uhc_env_reset: no clips loaded"; return -3; }
     CK(cudaSetDevice(e->device));
@@ -385,14 +394,20 @@ int uhc_env_reset(UhcEngine *e, int n, const int *env_ids_host, const int *clip_
     memcpy(e->h_ids, env_ids_host, n * sizeof(int)); memcpy(e->h_ids + n, clip_host, n * sizeof(int));
     memcpy(e->h_ids + 2 * n, start_host, n * sizeof(int)); memcpy(e->h_ids + 3 * n, len_host, n * sizeof(int));
     CK(cudaMemcpyAsync(e->d_ids, e->h_ids, (size_t)4 * n * sizeof(int), cudaMemcpyHostToDevice, st));
+    EngineView<float> evf = e->evf; EngineView<double> evd = e->evd;
+    if (no_auto_reset) { evf.cfg.auto_reset = 0; evd.cfg.auto_reset = 0; }
     if (e->precision == 32)
-        k_env_reset<float, EPB_F><<<(n + EPB_F - 1) / EPB_F, 32 * EPB_F, step_smem<float, EPB_F>(), st>>>(e->evf, n, e->d_ids, e->d_ids + n, e->d_ids + 2 * n, e->d_ids + 3 * n, qpos_dev, qvel_dev, obs_dev);
+        k_env_reset<float, EPB_F><<<(n + EPB_F - 1) / EPB_F, 32 * EPB_F, step_smem<float, EPB_F>(), st>>>(evf, n, e->d_ids, e->d_ids + n, e->d_ids + 2 * n, e->d_ids + 3 * n, qpos_dev, qvel_dev, obs_dev);
     else
-        k_env_reset<double, EPB_D><<<(n + EPB_D - 1) / EPB_D, 32 * EPB_D, step_smem<double, EPB_D>(), st>>>(e->evd, n, e->d_ids, e->d_ids + n, e->d_ids + 2 * n, e->d_ids + 3 * n, qpos_dev, qvel_dev, obs_dev);
+        k_env_reset<double, EPB_D><<<(n + EPB_D - 1) / EPB_D, 32 * EPB_D, step_smem<double, EPB_D>(), st>>>(evd, n, e->d_ids, e->d_ids + n, e->d_ids + 2 * n, e->d_ids + 3 * n, qpos_dev, qvel_dev, obs_dev);
     CK(cudaGetLastError());
     CK(cudaEventRecord(e->ids_done, st));
     e->launches++;
     return 0;
+}
+int uhc_env_reset(UhcEngine *e, int n, const int *env_ids_host, const int *clip_host, const int *start_host, const int *len_host,
+                  const float *qpos_dev, const float *qvel_dev, float *obs_dev, void *stream) {
+    return env_reset_impl(e, n, env_ids_host, clip_host, start_host, len_host, qpos_dev, qvel_dev, obs_dev, stream, false);
 }
 
 int uhc_env_step(UhcEngine *e, const float *actions_dev, float *obs_dev, float *reward_dev, float *cinfo_dev, int *fail_dev, int *end_dev,
@@ -403,9 +418,9 @@ int uhc_env_step(UhcEngine *e, const float *actions_dev, float *obs_dev, float *
     cudaStream_t st = (cudaStream_t)stream;
     if (e->d_order) { k_order_envs<<<1, 1024, 0, st>>>(e->precision == 32 ? e->evf.istate : e->evd.istate, e->E, e->d_order); e->launches++; }
     if (e->precision == 32)
-        k_env_step<float, EPB_F><<<(e->E + EPB_F - 1) / EPB_F, 32 * EPB_F, step_smem<float, EPB_F>(), st>>>(e->evf, actions_dev, obs_dev, reward_dev, cinfo_dev, fail_dev, end_dev, percent_dev, torque_dev, e->d_order);
+        k_env_step<float, EPB_F><<<(e->E + EPB_F - 1) / EPB_F, 32 * EPB_F, step_smem<float, EPB_F>(), st>>>(e->evf, actions_dev, obs_dev, reward_dev, cinfo_dev, fail_dev, end_dev, percent_dev, torque_dev, e->d_order, EvalView{});
     else
-        k_env_step<double, EPB_D><<<(e->E + EPB_D - 1) / EPB_D, 32 * EPB_D, step_smem<double, EPB_D>(), st>>>(e->evd, actions_dev, obs_dev, reward_dev, cinfo_dev, fail_dev, end_dev, percent_dev, torque_dev, e->d_order);
+        k_env_step<double, EPB_D><<<(e->E + EPB_D - 1) / EPB_D, 32 * EPB_D, step_smem<double, EPB_D>(), st>>>(e->evd, actions_dev, obs_dev, reward_dev, cinfo_dev, fail_dev, end_dev, percent_dev, torque_dev, e->d_order, EvalView{});
     CK(cudaGetLastError());
     e->launches++;
     return 0;
@@ -522,3 +537,32 @@ int uhc_engine_act_dim(const UhcEngine *e) { return e ? (e->precision == 32 ? e-
 int uhc_kernel_launches(const UhcEngine *e) { return e ? e->launches : -1; }
 
 }  // extern "C"
+
+// ---- internal entry points of the evaluation loop (eval_internal.h)
+int uhc_env_step_eval(UhcEngine *e, const float *actions_dev, float *obs_dev, float *reward_dev, int *fail_dev, int *end_dev, const EvalView &xv, cudaStream_t st) {
+    CK(cudaSetDevice(e->device));
+    // evaluation never re-seeds by sampling: the reactive standing-neutral starts of a training reset stay off (they need auto_reset)
+    if (e->precision == 32) {
+        EngineView<float> ev = e->evf; ev.cfg.auto_reset = 0;
+        k_env_step<float, EPB_F, true><<<(e->E + EPB_F - 1) / EPB_F, 32 * EPB_F, step_smem<float, EPB_F>(), st>>>(ev, actions_dev, obs_dev, reward_dev, e->d_cinfo, fail_dev, end_dev, e->d_pct, nullptr, nullptr, xv);
+    } else {
+        EngineView<double> ev = e->evd; ev.cfg.auto_reset = 0;
+        k_env_step<double, EPB_D, true><<<(e->E + EPB_D - 1) / EPB_D, 32 * EPB_D, step_smem<double, EPB_D>(), st>>>(ev, actions_dev, obs_dev, reward_dev, e->d_cinfo, fail_dev, end_dev, e->d_pct, nullptr, nullptr, xv);
+    }
+    CK(cudaGetLastError());
+    e->launches++;
+    return 0;
+}
+
+int uhc_env_reset_eval(UhcEngine *e, int n, const int *env_ids_host, const int *clip_host, const int *start_host, const int *len_host, float *obs_dev,
+                       cudaStream_t st) {
+    return env_reset_impl(e, n, env_ids_host, clip_host, start_host, len_host, nullptr, nullptr, obs_dev, st, true);
+}
+
+int uhc_engine_expert_table(const UhcEngine *e, EngineTable *out) {
+    if (!e->d_expert) { g_err = "no clips loaded"; return -3; }
+    out->expert = e->d_expert; out->clip_adr = e->d_clip_adr; out->precision = e->precision; out->num_clips = e->num_clips; out->device = e->device;
+    out->clip_len = e->clip_len_h.data();
+    out->trail_steps = e->precision == 32 ? e->evf.cfg.trail_steps : e->evd.cfg.trail_steps;
+    return 0;
+}

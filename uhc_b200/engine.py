@@ -148,6 +148,7 @@ class Engine:
     def close(self):
         if getattr(self, "h", None):
             self.lib.uhc_rollout_release(self.h)
+            self.lib.uhc_eval_release(self.h)
             self.lib.uhc_engine_destroy(self.h)
             self.h = None
 
