@@ -79,11 +79,15 @@ class AgentCopycat:
         if not torch.cuda.is_available():
             raise RuntimeError("the B200 engine needs a CUDA device (the reference's CPU sampling path is replaced, not kept as a fallback)")
         self.model_tables = HumanoidModel()
+        # extra key motion_lib: "host" (expert tables from uhc_b200.motion_lib, packed and uploaded) | "device" (built on the GPU from the
+        # raw SMPL sequences, Engine.load_smpl_clips)
+        self.motion_lib = str(cfg.get("motion_lib", "host"))
+        assert self.motion_lib in ("host", "device"), "motion_lib: host | device"
         # data (setup_data_loader :128-134)
-        self.data_loader = DatasetAMASSSingle(cfg.data_specs, data_mode="train", model=self.model_tables)
+        self.data_loader = DatasetAMASSSingle(cfg.data_specs, data_mode="train", model=self.model_tables, motion_lib=self.motion_lib)
         self.test_data_loaders = [self.data_loader]
         if len(cfg.data_specs.get("test_file_path", [])) > 0:
-            self.test_data_loaders.append(DatasetAMASSSingle(cfg.data_specs, data_mode="test", model=self.model_tables))
+            self.test_data_loaders.append(DatasetAMASSSingle(cfg.data_specs, data_mode="test", model=self.model_tables, motion_lib=self.motion_lib))
         self.freq_dict = {k: [] for k in self.data_loader.data_keys}
         rw = cfg.reward_weights or {}
         w = [rw.get(k, d) for k, d in (("w_p", 0.6), ("w_v", 0.1), ("w_e", 0.2), ("w_c", 0.1), ("w_vf", 0.0))]
@@ -99,7 +103,7 @@ class AgentCopycat:
             sync = make_nccl_grad_sync(world)
         rfc_mode = supported_variant(cfg)       # refuses (AssertionError) what the batched engine does not implement instead of accepting it silently (ADVICE r1)
         self.agent = BatchedAgent(
-            self.num_envs, self.data_loader.experts, self.data_loader.shapes, device=dev_index, seed=cfg.seed, policy_hsize=cfg.policy_hsize,
+            self.num_envs, self.data_loader.smpl_clips() if self.motion_lib == "device" else self.data_loader.experts, self.data_loader.shapes, device=dev_index, seed=cfg.seed, policy_hsize=cfg.policy_hsize,
             value_hsize=cfg.value_hsize, htype=cfg.policy_htype, log_std=cfg.log_std, policy_lr=cfg.policy_lr, value_lr=cfg.value_lr,
             gamma=cfg.gamma, tau=cfg.tau, clip_epsilon=cfg.clip_epsilon, num_optim_epoch=cfg.num_optim_epoch, grad_clip=40.0,
             t_min=cfg.data_specs.get("t_min", 90), t_max=cfg.data_specs.get("t_max", -1), rank=rank, world=world, grad_sync=sync,
@@ -207,7 +211,7 @@ class AgentCopycat:
         for loader in self.test_data_loaders:
             n = loader.get_len()
             if loader is not self.data_loader:
-                eng.load_clips(loader.experts, loader.shapes)      # invalidates every env record: evaluate resets the slots it runs
+                self._load_tables(loader)      # invalidates every env record: evaluate resets the slots it runs
             eng.set_cfg(**self._env_cfg(test=True))
             ev = self.agent.evaluate(0, n, bool(cfg.fail_safe))
             res = {}
@@ -228,7 +232,7 @@ class AgentCopycat:
                 if k in self.freq_dict:      # eval outcome feeds the failure-weighted sampler like a training episode ([percent, fr_start])
                     self.freq_dict[k] = (self.freq_dict[k] + [[1.0 if m["succ"][0] else min(percent, 0.999), 0]])[-self.max_freq:]
             if loader is not self.data_loader:
-                eng.load_clips(self.data_loader.experts, self.data_loader.shapes)
+                self._load_tables(self.data_loader)
             eng.set_cfg(**self._env_cfg(test=False))
             self.agent.obs = None
             names = ("succ", "reward", "mpjpe", "mpjpe_g", "pa_mpjpe", "accel_dist", "vel_dist", "root_dist")
@@ -243,6 +247,14 @@ class AgentCopycat:
                 joblib.dump(res, path)
         self._push_clip_weights()
         return res_dicts
+
+    def _load_tables(self, loader):
+        eng = self.agent.engine
+        if self.motion_lib == "device":
+            c = loader.smpl_clips()
+            eng.load_smpl_clips(c["pose_aa"], c["trans"], loader.shapes)
+        else:
+            eng.load_clips(loader.experts, loader.shapes)
 
     def _env_cfg(self, test):
         cfg = self.cfg

@@ -1,6 +1,7 @@
 """DatasetAMASSSingle of the reference (uhc/data_loaders/dataset_amass_single.py:27-253): same pickle schema
 {key: {pose_aa, pose_6d, trans, beta, gender, ...}}, same filtering (len >= t_min + 1), same sampling rules; in addition it
-precomputes the expert tables of every clip once (uhc_b200.motion_lib) instead of once per episode."""
+precomputes the expert tables of every clip once (uhc_b200.motion_lib) instead of once per episode.  With motion_lib="device" the engine builds
+the tables from the raw sequences (smpl_clips(), Engine.load_smpl_clips) and the host tables are computed only if `experts` is read."""
 import random
 
 import joblib
@@ -17,7 +18,7 @@ def _gender_code(g):
 
 
 class DatasetAMASSSingle:
-    def __init__(self, data_specs, data_mode="train", model=None):
+    def __init__(self, data_specs, data_mode="train", model=None, motion_lib="host"):
         np.random.seed(0)
         random.seed(0)
         self.data_root = data_specs["file_path"] if data_mode == "train" else data_specs["test_file_path"]
@@ -43,9 +44,25 @@ class DatasetAMASSSingle:
             self.sample_keys += [(k, [-1])] * reps
         self.seq_len = len(self.data_keys)
         self.curr_key = ""
-        # expert tables of every clip, once (humanoid_im.py:182-215 does this per episode)
-        self.experts = [motion_lib.make_expert(self.data["pose_aa"][k], self.data["trans"][k], model) for k in self.data_keys]
         self.shapes = [np.concatenate([self.data["beta"][k][0], [self.data["gender"][k][0]]]) for k in self.data_keys]
+        assert motion_lib in ("host", "device"), "motion_lib: host | device"
+        self._model, self._experts = model, None
+        if motion_lib == "host":
+            self._experts = self._make_experts()
+
+    def _make_experts(self):
+        # expert tables of every clip, once (humanoid_im.py:182-215 does this per episode)
+        return [motion_lib.make_expert(self.data["pose_aa"][k], self.data["trans"][k], self._model) for k in self.data_keys]
+
+    @property
+    def experts(self):
+        if self._experts is None:
+            self._experts = self._make_experts()
+        return self._experts
+
+    def smpl_clips(self):
+        """the raw sequences of every clip in data_keys order, as BatchedAgent / Engine.load_smpl_clips take them"""
+        return {"pose_aa": [self.data["pose_aa"][k] for k in self.data_keys], "trans": [self.data["trans"][k] for k in self.data_keys]}
 
     def get_len(self):
         return self.seq_len

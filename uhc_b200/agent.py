@@ -118,7 +118,12 @@ class BatchedAgent:
         self.auto_reset = bool(env_cfg.pop("auto_reset", True))
         self.engine = Engine(num_envs, model=model, device=device, precision=precision, variants=variants, auto_reset=int(self.auto_reset), t_min=t_min, t_max=t_max,
                              reset_seed=seed * 7919 + rank * 104729 + 1, **env_cfg)
-        self.engine.load_clips(clips, shapes, clip_models)   # clip_models: body-shape variant per clip (the reference rebuilds the robot per clip)
+        # clips: expert dicts (host motion library) or {"pose_aa": [...], "trans": [...]} raw SMPL sequences whose tables are built on the device;
+        # clip_models: body-shape variant per clip (the reference rebuilds the robot per clip)
+        if isinstance(clips, dict):
+            self.engine.load_smpl_clips(clips["pose_aa"], clips.get("trans"), shapes, clip_models)
+        else:
+            self.engine.load_clips(clips, shapes, clip_models)
         self.sampler = ClipSampler(self.engine.clip_len, t_min, t_max, seed=seed * 9973 + rank)
         A = self.act_dim = self.engine.act_dim          # env.action_dim (humanoid_im.py:250): 69 + (6 | 216) + (30 if meta_pd)
         D = self.obs_dim = self.engine.obs_dim          # env.obs_dim: 657 (obs v2) or 784 (obs v1)

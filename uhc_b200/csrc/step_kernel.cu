@@ -12,6 +12,7 @@
 #endif
 #include "env_step.h"
 #include "eval_internal.h"
+#include "clip_table.h"
 
 using namespace uhc;
 
@@ -147,6 +148,8 @@ struct UhcEngine {
     std::vector<float> clip_w;            // clip sampling weights behind clip_cdf (uhc_set_clip_weights), empty = sample_keys rule
     int *d_order = nullptr;   // warp slot -> environment (work-sorted each step), null = identity
     std::vector<int> clip_len_h;   // host copy of the clip lengths (argument validation)
+    std::vector<double> kin_h;     // [nshape][24][6] body offsets and centres of mass, fp64 (the device motion library's FK)
+    std::vector<int> kin_i;        // parent [24], end-effector bodies [5]
 };
 
 template <class T> static int dev_copy(UhcEngine *e, T **dst, const T *src, size_t n) {
@@ -226,6 +229,9 @@ int uhc_engine_create(const UhcModelHost *model, const UhcEnvCfg *cfg, int num_e
     e->E = num_envs; e->device = device; e->precision = precision; e->launches = 0; e->nshape = model->nshape > 0 ? model->nshape : 1;
     int rc = precision == 32 ? build_view<float>(e, e->evf, model, cfg) : build_view<double>(e, e->evd, model, cfg);
     if (rc) { delete e; return rc; }
+    e->kin_h.resize((size_t)e->nshape * NB * 6);
+    for (int v = 0; v < e->nshape; v++) for (int b = 0; b < NB; b++) for (int k = 0; k < 6; k++) e->kin_h[((size_t)v * NB + b) * 6 + k] = model->body_f[((size_t)v * NB + b) * BODYF + k];
+    e->kin_i.assign(model->parent, model->parent + NB); e->kin_i.insert(e->kin_i.end(), model->ee, model->ee + 5);
     {   // work-sorted warp slots: opt-in (UHC_SORT_ENVS=1).  Measured at 4096 envs: 1.52 M env-steps/s sorted vs 1.57 M with the identity
         // mapping -- the previous step's iteration total does not predict the per-substep imbalance well enough to pay for itself
         const char *se = getenv("UHC_SORT_ENVS");
@@ -303,33 +309,21 @@ int uhc_load_clips(UhcEngine *e, int nclips, const int *clip_len, const double *
     if (!e || nclips <= 0 || !clip_len || !frames_host || !shape_host) { g_err = "uhc_load_clips: bad argument"; return -2; }
     CK(cudaSetDevice(e->device));
     CK(cudaDeviceSynchronize());
-    std::vector<int> adr(nclips + 1, 0);
-    for (int i = 0; i < nclips; i++) { if (clip_len[i] < 2) { g_err = "uhc_load_clips: clip shorter than 2 frames"; return -2; } adr[i + 1] = adr[i] + clip_len[i]; }
-    const size_t nf = (size_t)adr[nclips] * EX_SIZE, ns = (size_t)nclips * 17;
-    if (e->d_expert) { cudaFree(e->d_expert); cudaFree(e->d_shape); cudaFree(e->d_clip_adr); cudaFree(e->d_clip_cdf); e->d_expert = e->d_shape = nullptr; e->d_clip_adr = nullptr; e->d_clip_cdf = nullptr; }
-    CK(cudaMalloc((void **)&e->d_clip_adr, (nclips + 1) * sizeof(int)));
-    CK(cudaMemcpy(e->d_clip_adr, adr.data(), (nclips + 1) * sizeof(int), cudaMemcpyHostToDevice));
-    e->num_clips = nclips; e->clip_len_h.assign(clip_len, clip_len + nclips); e->clip_w.clear();
-    e->evf.cfg.num_clips = nclips; e->evd.cfg.num_clips = nclips;
-    if (upload_clip_cdf(e)) return -1;
-    if (e->d_clip_model) { cudaFree(e->d_clip_model); e->d_clip_model = nullptr; }
-    e->evf.clip_model = nullptr; e->evd.clip_model = nullptr;
-    // every env record points into the OLD clip table: invalidate them all (len = 0); the step kernel skips (and flags) an env
-    // until uhc_env_reset gives it a slice of the new table
-    CK(cudaMemset(e->precision == 32 ? e->evf.istate : e->evd.istate, 0, (size_t)e->E * SI_SIZE * sizeof(int)));
+    size_t total = 0;
+    for (int i = 0; i < nclips; i++) { if (clip_len[i] < 2) { g_err = "uhc_load_clips: clip shorter than 2 frames"; return -2; } total += clip_len[i]; }
+    const size_t nf = total * EX_SIZE, ns = (size_t)nclips * 17;
+    void *d_expert = nullptr, *d_shape = nullptr;
     if (e->precision == 32) {
         std::vector<float> f(nf), s(ns);
         for (size_t i = 0; i < nf; i++) f[i] = (float)frames_host[i];
         for (size_t i = 0; i < ns; i++) s[i] = (float)shape_host[i];
-        CK(cudaMalloc(&e->d_expert, nf * 4)); CK(cudaMalloc(&e->d_shape, ns * 4));
-        CK(cudaMemcpy(e->d_expert, f.data(), nf * 4, cudaMemcpyHostToDevice)); CK(cudaMemcpy(e->d_shape, s.data(), ns * 4, cudaMemcpyHostToDevice));
-        e->evf.expert = (const float *)e->d_expert; e->evf.clip_shape = (const float *)e->d_shape; e->evf.clip_adr = e->d_clip_adr;
+        CK(cudaMalloc(&d_expert, nf * 4)); CK(cudaMalloc(&d_shape, ns * 4));
+        CK(cudaMemcpy(d_expert, f.data(), nf * 4, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_shape, s.data(), ns * 4, cudaMemcpyHostToDevice));
     } else {
-        CK(cudaMalloc(&e->d_expert, nf * 8)); CK(cudaMalloc(&e->d_shape, ns * 8));
-        CK(cudaMemcpy(e->d_expert, frames_host, nf * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(e->d_shape, shape_host, ns * 8, cudaMemcpyHostToDevice));
-        e->evd.expert = (const double *)e->d_expert; e->evd.clip_shape = (const double *)e->d_shape; e->evd.clip_adr = e->d_clip_adr;
+        CK(cudaMalloc(&d_expert, nf * 8)); CK(cudaMalloc(&d_shape, ns * 8));
+        CK(cudaMemcpy(d_expert, frames_host, nf * 8, cudaMemcpyHostToDevice)); CK(cudaMemcpy(d_shape, shape_host, ns * 8, cudaMemcpyHostToDevice));
     }
-    return 0;
+    return uhc_engine_install_clips(e, nclips, clip_len, d_expert, d_shape);
 }
 
 int uhc_set_neutral_pose(UhcEngine *e, const double *qpos76, const double *qvel75) {
@@ -566,3 +560,33 @@ int uhc_engine_expert_table(const UhcEngine *e, EngineTable *out) {
     out->trail_steps = e->precision == 32 ? e->evf.cfg.trail_steps : e->evd.cfg.trail_steps;
     return 0;
 }
+
+int uhc_engine_install_clips(UhcEngine *e, int nclips, const int *clip_len, void *expert_dev, void *shape_dev) {
+    CK(cudaSetDevice(e->device));
+    CK(cudaDeviceSynchronize());      // in-flight work may still read the old table
+    std::vector<int> adr(nclips + 1, 0);
+    for (int i = 0; i < nclips; i++) adr[i + 1] = adr[i] + clip_len[i];
+    if (e->d_expert) { cudaFree(e->d_expert); cudaFree(e->d_shape); cudaFree(e->d_clip_adr); cudaFree(e->d_clip_cdf); e->d_expert = e->d_shape = nullptr; e->d_clip_adr = nullptr; e->d_clip_cdf = nullptr; }
+    e->d_expert = expert_dev; e->d_shape = shape_dev;
+    CK(cudaMalloc((void **)&e->d_clip_adr, (nclips + 1) * sizeof(int)));
+    CK(cudaMemcpy(e->d_clip_adr, adr.data(), (nclips + 1) * sizeof(int), cudaMemcpyHostToDevice));
+    e->num_clips = nclips; e->clip_len_h.assign(clip_len, clip_len + nclips); e->clip_w.clear();
+    e->evf.cfg.num_clips = nclips; e->evd.cfg.num_clips = nclips;
+    if (upload_clip_cdf(e)) return -1;
+    if (e->d_clip_model) { cudaFree(e->d_clip_model); e->d_clip_model = nullptr; }
+    e->evf.clip_model = nullptr; e->evd.clip_model = nullptr;
+    // every env record points into the OLD clip table: invalidate them all (len = 0); the step kernel skips (and flags) an env
+    // until uhc_env_reset gives it a slice of the new table
+    CK(cudaMemset(e->precision == 32 ? e->evf.istate : e->evd.istate, 0, (size_t)e->E * SI_SIZE * sizeof(int)));
+    if (e->precision == 32) { e->evf.expert = (const float *)e->d_expert; e->evf.clip_shape = (const float *)e->d_shape; e->evf.clip_adr = e->d_clip_adr; }
+    else { e->evd.expert = (const double *)e->d_expert; e->evd.clip_shape = (const double *)e->d_shape; e->evd.clip_adr = e->d_clip_adr; }
+    return 0;
+}
+
+int uhc_engine_kin(const UhcEngine *e, EngineKin *out) {
+    out->off_ipos = e->kin_h.data(); out->parent = e->kin_i.data(); out->ee = e->kin_i.data() + NB;
+    out->nshape = e->nshape; out->precision = e->precision; out->device = e->device;
+    return 0;
+}
+
+void uhc_engine_set_error(const char *msg) { g_err = msg; }

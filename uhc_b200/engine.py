@@ -177,6 +177,36 @@ class Engine:
         if clip_models is not None:
             _chk(self.lib.uhc_set_clip_models(self.h, C.c_int(len(experts)), _ip(clip_models)))
 
+    def load_smpl_clips(self, pose_aa, trans, shapes=None, clip_models=None):
+        """expert tables built on the device from raw SMPL sequences (uhc_load_clips_smpl, include/uhc_motion.h): the records
+        make_expert + load_clips would give, without any host expert dict.  pose_aa: per-clip [T][72] or [T][156] axis-angle arrays (one width
+        for all clips); trans: per-clip [T][3] arrays (a None entry, or trans None, = the default root height); shapes: [C][17]; clip_models:
+        body-shape variant per clip."""
+        pose = [np.asarray(p, dtype=np.float64) for p in pose_aa]
+        n = len(pose)
+        widths = {p.shape[1] for p in pose}
+        if len(widths) != 1:
+            raise ValueError(f"load_smpl_clips: every clip needs the same pose width, got {sorted(widths)}")
+        lens = np.array([len(p) for p in pose], np.int32)
+        tr = None
+        if trans is not None and any(t is not None for t in trans):
+            tr = np.ascontiguousarray(np.concatenate([np.asarray(t, dtype=np.float64).reshape(len(p), 3) if t is not None
+                                                      else np.tile([0.0, 0.0, 0.91437225], (len(p), 1)) for p, t in zip(pose, trans)]))
+        frames = np.ascontiguousarray(np.concatenate(pose))
+        shp = np.ascontiguousarray(np.zeros((n, 17)) if shapes is None else np.asarray(shapes, dtype=np.float64).reshape(n, 17))
+        cm = None if clip_models is None else np.ascontiguousarray(clip_models, dtype=np.int32)
+        d = lambda a: a.ctypes.data_as(C.POINTER(C.c_double))
+        _chk(self.lib.uhc_load_clips_smpl(self.h, C.c_int(n), _ip(lens), C.c_int(widths.pop()), d(frames), d(tr) if tr is not None else None, d(shp),
+                                          cm.ctypes.data_as(C.POINTER(C.c_int)) if cm is not None else None))
+        self.clip_len = lens
+
+    def get_clip_frames(self, frame0=0, nframes=None):
+        """rows of the device clip table (all clips concatenated) as [n][576] doubles (uhc_get_clip_frames)"""
+        n = int(self.clip_len.sum()) - frame0 if nframes is None else int(nframes)
+        out = np.empty((n, EX_SIZE))
+        _chk(self.lib.uhc_get_clip_frames(self.h, C.c_int(frame0), C.c_int(n), out.ctypes.data_as(C.POINTER(C.c_double))))
+        return out
+
     def _stream(self):
         return C.c_void_p(self.torch.cuda.current_stream(self.device).cuda_stream)
 
